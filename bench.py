@@ -5,6 +5,10 @@
   python bench.py --impl reference --steps K --warmup W    the reference algorithm on the host CPU cores
                                                            (oracle port: the Rust reference cannot be built here)
   python bench.py --workload C1|C2|C3|C4|C5 [--series n]   the other BASELINE shapes (default C4, the headline)
+  python bench.py ... --dump-outputs DIR                   also write what the last timed step computed, DIR/<name>.npy
+                                                           (inputs are seeded: the same arguments give the same inputs;
+                                                           f64 sums / means may differ in the last bits between runs
+                                                           as the device adds in varying order, compare within 1e-6)
 
 Workload C4 (config.workload, the configuration BASELINE's metric is quoted on): 1 000 000 series x 1 000 points,
 mixed i64 (Delta/simple8b) and f64 (Gorilla, full-mantissa) columns, 20 % of the series with jittered timestamps
@@ -265,8 +269,8 @@ def cpu_arm(arena, descs, query, steps, warmup, max_s=150.0):
     """Times the oracle (port of the reference algorithm; CRC32 of every page verified on every read like
     Page::crc_validation) on the WHOLE workload: all selected series, every step. The page set is opened once
     (series index + persistent worker pool, like the reference's cached TsmReader metadata and live runtime threads);
-    a step is one query. Steps are cut short only if the run would exceed max_s seconds (stated in `sample`).
-    Returns (info, result, seconds per step)."""
+    a step is one query. Steps are cut short only if the run would exceed max_s seconds (stated in `sample`; None:
+    never). Returns (info, result of the last step, seconds per step)."""
     from oracle import pyoracle as orc
     cores = host_threads()
     op = orc.OpenPages(arena, descs, cores)
@@ -278,7 +282,7 @@ def cpu_arm(arena, descs, query, steps, warmup, max_s=150.0):
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
-        if time.perf_counter() - t_begin + dt > max_s and len(times) >= 2:
+        if max_s is not None and time.perf_counter() - t_begin + dt > max_s and len(times) >= 2:
             break
     op.close()
     med = float(np.median(times))
@@ -307,6 +311,48 @@ def results_match(got, exp):
     return bool(ok)
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def result_arrays(res):
+    """ScanResult -> {name: array} as a caller reads it: per output column c<id>_<agg> the typed values as float64
+    ([n_groups, n_buckets], 0 where invalid) and c<id>_<agg>_valid as float32 0 / 1."""
+    out = {}
+    for col, agg in res.names:
+        v, ok = res.column(col, agg)
+        out["c%d_%s" % (col, agg)] = v.astype(np.float64)
+        out["c%d_%s_valid" % (col, agg)] = ok.astype(np.float32)
+    return out
+
+
+def decoded_arrays(pages):
+    """[(u64 values, validity)] of decode_pages -> {name: array}, like result_arrays. float64 cannot hold a nanosecond
+    timestamp exactly, so each 64-bit value is written as its high and low 32-bit halves."""
+    out = {}
+    for i, (v, ok) in enumerate(pages):
+        out["page%d_values_hi" % i] = (v >> np.uint64(32)).astype(np.float64)
+        out["page%d_values_lo" % i] = (v & np.uint64(0xFFFFFFFF)).astype(np.float64)
+        out["page%d_valid" % i] = ok.astype(np.float32)
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy. Above DUMP_MAX_BYTES in all, each array is cut to the same share of
+    its elements at positions drawn by a fixed seed (flattened, in order), so arrays of one shape keep the same
+    positions and two runs with the same arguments compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    share = min(1.0, (DUMP_MAX_BYTES - 256 * len(arrays)) / max(total, 1))  # 256: room for each .npy header
+    for name, a in arrays.items():
+        if share < 1.0:
+            flat = a.reshape(-1)
+            keep = np.sort(np.random.default_rng(0).choice(flat.size, int(flat.size * share), replace=False))
+            a = flat[keep]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print("bench: wrote %d arrays to %s%s" % (len(arrays), out_dir, "" if share == 1.0 else
+                                              " (seeded sample: %.4f of the elements)" % share), file=sys.stderr)
+
+
 def bench_decode_only(args, rank, world):
     """C1: 1 series x 10 000 i64 points (Delta + simple8b), decode only - tskvgpu_decode_pages vs the oracle's
     column decode (the reference's own CPU bench shape). Single GPU."""
@@ -317,7 +363,7 @@ def bench_decode_only(args, rank, world):
     n_pts = 10_000 * 2  # the time page and the value page
     cores = 1
     times = []
-    for i in range(args.warmup + max(args.steps, 20)):
+    for i in range(args.warmup + args.steps):
         t0 = time.perf_counter()
         exp = orc.decode_pages(g.arena, g.descs)
         if i >= args.warmup:
@@ -325,6 +371,8 @@ def bench_decode_only(args, rank, world):
     cpu = {"value": n_pts / float(np.median(times)), "unit": "points/s", "cores": cores, "kind": "port",
            "sample": "both pages of the series, every step, 1 thread (a single series is one task in the reference)"}
     if args.impl == "reference":
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, decoded_arrays(exp))
         print(json.dumps({"impl": "reference", "metric": "decoded points/s", "value": cpu["value"], "unit": "points/s",
                           "n_gpus": args.gpus, "steps": len(times), "warmup": args.warmup,
                           "ms_per_step": float(np.median(times)) * 1e3, "higher_is_better": True, "scaling": "strong",
@@ -335,7 +383,7 @@ def bench_decode_only(args, rank, world):
     eng = Engine(int(os.environ.get("LOCAL_RANK", "0")))
     pages = eng.upload_pages(g.arena, g.descs)
     dev_ms, e2e = [], []
-    for i in range(args.warmup + max(args.steps, 20)):
+    for i in range(args.warmup + args.steps):
         t0 = time.perf_counter()
         got = eng.decode_pages(pages, g.descs)
         dt = time.perf_counter() - t0
@@ -343,6 +391,8 @@ def bench_decode_only(args, rank, world):
             e2e.append(dt)
             dev_ms.append(eng.counters()["elapsed_scan_ms"])
     ok = all((gm == em).all() and (gv[em] == ev[em]).all() for (gv, gm), (ev, em) in zip(got, exp))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, decoded_arrays(got))
     page_bytes = int(g.descs["size"].sum())
     peak = 6584.5
     try:
@@ -373,7 +423,11 @@ def main():
     ap.add_argument("--workload", default="C4", choices=["C1", "C2", "C3", "C4", "C5"])
     ap.add_argument("--series", type=int, default=0, help="total series (default: the workload's BASELINE size)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/<name>.npy (float64 / float32, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -391,7 +445,9 @@ def main():
         n_ref = min(n_series, 1_000_000)  # a C5-sized page set does not fit host memory comfortably: bounded
         g = wl.generate(0, n_ref)
         sel = wl.select(n_ref)
-        info, _, step_s = cpu_arm(g.arena, g.descs, wl.query(sel), steps, args.warmup)
+        info, res, step_s = cpu_arm(g.arena, g.descs, wl.query(sel), steps, args.warmup, max_s=None)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, result_arrays(res))
         if n_ref != n_series:
             info["sample"] = "first %d of %d series; " % (n_ref, n_series) + info["sample"]
         line = {"impl": "reference", "metric": METRIC, "value": info["value"], "unit": "points/s",
@@ -464,6 +520,8 @@ def main():
     dev_ms = timed_steps(scan, exchange, steps)
     barrier()
     clocks = sampler.stop(t_region, time.perf_counter()) if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # finalize() re-reads the last step's state; the roofline runs below overwrite it
+        dump_outputs(args.dump_outputs, result_arrays(scan.finalize()))
     t = torch.tensor([dev_ms, float(points_local)], dtype=torch.float64, device=device)
     if world > 1:
         tmax = t.clone()
